@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- body-steps/sec of the Edyn per-step hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b2d|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b2d|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one fixed simulation step (broadphase -> narrowphase -> islands -> solve -> integrate) of the whole scene.
 
@@ -340,6 +340,19 @@ def traffic_for(name):
     return None
 
 
+DUMP_MAX_BODIES = 1 << 18      # per workload: 13 floats a body, so the four workloads stay far below 64 MB
+
+
+def dump_outputs(out_dir, name, state):
+    """Writes the body state a caller of b2d_step receives (pos, orn, linvel, angvel) as out_dir/<workload>.<field>.npy,
+    float32.  A workload with more bodies than DUMP_MAX_BODIES is sampled: the same seeded, sorted body indices every run."""
+    n = len(state["pos"])
+    idx = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_BODIES, replace=False)) if n > DUMP_MAX_BODIES else np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    for k in ("pos", "orn", "linvel", "angvel"):
+        np.save(os.path.join(out_dir, f"{name}.{k}.npy"), np.ascontiguousarray(state[k][idx], np.float32))
+
+
 def measure_single(args, name, local_rank, steps, warmup, cpu_seconds, sample_clocks, real_reference=False):
     """One workload, whole scene on one GPU: device-resident value, e2e through host buffers, roofline, CPU baseline."""
     import torch
@@ -377,7 +390,9 @@ def measure_single(args, name, local_rank, steps, warmup, cpu_seconds, sample_cl
     pinned = {k: torch.empty((n_all, d), dtype=torch.float32).pin_memory() for k, d in (("pos", 3), ("orn", 4), ("linvel", 3), ("angvel", 3))}
     host = {k: v.numpy() for k, v in pinned.items()}
     w.download_state(aabb=False, out=host)
-    e2e_steps = max(3, min(steps, 50))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, name, host)
+    e2e_steps = steps
     for _ in range(3):
         w.upload_state(host["pos"], host["orn"], host["linvel"], host["angvel"])
         w.step(1)
@@ -542,7 +557,7 @@ def run_sharded(args, world_size, rank, local_rank):
     pinned = {k: torch.empty((n_loc, d), dtype=torch.float32).pin_memory() for k, d in (("pos", 3), ("orn", 4), ("linvel", 3), ("angvel", 3))}
     host = {k: v.numpy() for k, v in pinned.items()}
     w.download_state(aabb=False, out=host)
-    e2e_steps = max(3, min(args.steps, 50))
+    e2e_steps = args.steps
     for _ in range(3):
         w.upload_state(host["pos"], host["orn"], host["linvel"], host["angvel"])
         sw.step(1)
@@ -631,7 +646,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--ref-child", default=None, help=argparse.SUPPRESS)
     ap.add_argument("--exact-exchange", action="store_true", help="N > 1: read every step's rank boxes before the next step starts (no look-ahead margin)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="N = 1, device arm: after the timed steps write each workload's body state as DIR/<workload>.<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b2d" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl b2d --gpus 1")
     if args.ref_child:
         ref_child(args.ref_child)
         return

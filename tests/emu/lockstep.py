@@ -119,23 +119,24 @@ def lockstep_with_mutations(E, O, scene, steps, seed):
     return dict(ok=flags == 0, worst=0.0, points=events, flags=flags)
 
 
-def free_run_against_real_stepper(E, O):
-    """No oracle in between: the kernels (emulated) and the reference's real stepper, both free-running from the same scene.
-    Hinge chains are insensitive to the sweep order (tiny islands at rest), so the two must simply agree; hello_world must be
-    identical while the box falls."""
+def free_run_against_real_stepper(E):
+    """No oracle in between: the kernels (emulated) and the reference's real stepper (its states recorded by
+    tests/golden/make_ref_runs.py), both free-running from the same scene.  Hinge chains are insensitive to the sweep order
+    (tiny islands at rest), so the two must simply agree; hello_world must be identical while the box falls."""
     import numpy as np
-    from tests.golden import make_whole_step as G
+    from tests.golden import make_ref_runs as R
+    runs = np.load(R.OUT)
     out = []
-    for name, scene, marks in (("chains_64", E.scenes.hinge_chains(4, 4), (60, 300)), ("hello_world", E.scenes.hello_world(), (24,))):
-        st = scene["settings"]
+    for name, key in (("chains_64", "chains_4x4"), ("hello_world", "hello_world")):
+        fn, a, marks = R.FREE_RUNS[key]
+        scene = getattr(E.scenes, fn)(*a)
         w = E.scenes.build_world(scene)
-        r = O.RefWorld(vel_iters=st["velocity_iterations"], pos_iters=st["position_iterations"])
-        G.populate(r, scene)
         n, done = scene["dynamic"], 0
         for m in marks:
-            w.step(m - done); r.step(m - done); done = m
-            g, c = w.download_state(), r.state()
-            out.append(dict(scene=name, step=m, dpos=float(np.abs(g["pos"][:n] - c["pos"][:n]).max()), dvel=float(np.abs(g["linvel"][:n] - c["linvel"][:n]).max())))
+            w.step(m - done); done = m
+            g = w.download_state()
+            c = {k: runs[f"{key}.{m}.{k}"] for k in ("pos", "linvel")}
+            out.append(dict(scene=name, step=m, dpos=float(np.abs(g["pos"][:n] - c["pos"]).max()), dvel=float(np.abs(g["linvel"][:n] - c["linvel"]).max())))
         w.close()
     return out
 
@@ -156,7 +157,7 @@ def main():
              lambda: E.scenes.mixed_pile(5, jitter=0.01), lambda: E.scenes.hinge_chains(2, 2)]
     out, t0 = [], time.time()
     if kind == "vsref":
-        print(json.dumps(dict(results=free_run_against_real_stepper(E, O), seconds=0.0)))
+        print(json.dumps(dict(results=free_run_against_real_stepper(E), seconds=0.0)))
         return
     for i in range(first, last):
         scene = fixed[i]() if kind == "fixed" else (random_scene_wide if kind == "wide" else random_scene)(E, O, i)

@@ -71,11 +71,9 @@ def test_emulated_kernels_under_user_interference(O):
 
 
 def test_emulated_kernels_against_the_real_stepper_directly(O):
-    """Kernels (emulated) vs the reference's real stepper_sequential, both free-running, nothing replayed: the hinge-chain
-    family (config 5) within 1e-6 after 300 steps (measured 5e-10; north_star asks for 1e-4 relative after 1000), hello_world
-    identical during the fall."""
-    if O.ref_stepper() is None:
-        pytest.skip("oracle/_ref/libedyn_stepper.so not available")
+    """Kernels (emulated) vs the reference's real stepper_sequential (states recorded in tests/golden/ref_runs.npz), both
+    free-running, nothing replayed: the hinge-chain family (config 5) within 1e-6 after 300 steps (measured 5e-10;
+    north_star asks for 1e-4 relative after 1000), hello_world identical during the fall."""
     for res in _run("vsref", 0, 0):
         if res["scene"] == "hello_world":
             assert res["dpos"] == 0.0 and res["dvel"] == 0.0, res

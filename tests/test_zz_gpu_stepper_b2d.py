@@ -8,6 +8,7 @@ the reference is (tests/integration/Makefile) and shipped; the CPU suite exercis
 import numpy as np
 import pytest
 
+from tests.golden import make_ref_runs as R
 from tests.golden import make_whole_step as G
 from tests.test_stepper_b2d import EdynB2dWorld, _contacts_by_pair, build_integration, load
 
@@ -86,23 +87,20 @@ def test_device_binding_follows_the_real_cpu_stepper(dev, E, O):
     w.close()
 
 
-def test_device_chains_follow_the_real_stepper_free_running(gpu, E, O):
-    """No oracle in between: the B200 and the reference's real stepper_sequential, both free-running for 1000 steps on a
-    slice of config 5 (64 chains): the hinge-chain family is insensitive to the sweep order, so north_star's 1e-4 must
-    simply hold (5e-10 absolute under the CPU emulation of the kernels after 300 steps)."""
-    if O.ref_stepper() is None:
-        pytest.skip("oracle/_ref/libedyn_stepper.so not shipped")
+def test_device_chains_follow_the_real_stepper_free_running(gpu, E):
+    """No oracle in between: the B200 and the reference's real stepper_sequential (its end state recorded by
+    tests/golden/make_ref_runs.py), both free-running for 1000 steps on a slice of config 5 (64 chains): the hinge-chain
+    family is insensitive to the sweep order, so north_star's 1e-4 must simply hold (5e-10 absolute under the CPU
+    emulation of the kernels after 300 steps)."""
+    runs = np.load(R.OUT)
     scene = E.scenes.hinge_chains(8, 8)
-    st = scene["settings"]
     w = E.scenes.build_world(scene)
-    r = O.RefWorld(vel_iters=st["velocity_iterations"], pos_iters=st["position_iterations"])
-    G.populate(r, scene)
     n = scene["dynamic"]
-    w.step(1000); r.step(1000)
-    g, c = w.download_state(aabb=False), r.state()
-    rel = float(np.abs(g["pos"][:n] - c["pos"][:n]).max() / np.abs(c["pos"][:n]).max())
+    w.step(1000)
+    g, c = w.download_state(aabb=False), {k: runs[f"chains_8x8.1000.{k}"] for k in ("pos", "linvel")}
+    rel = float(np.abs(g["pos"][:n] - c["pos"]).max() / np.abs(c["pos"]).max())
     assert rel <= 1e-4, f"relative position error after 1000 steps {rel:.3e}"
-    assert float(np.abs(g["linvel"][:n] - c["linvel"][:n]).max()) <= 1e-3
+    assert float(np.abs(g["linvel"][:n] - c["linvel"]).max()) <= 1e-3
     w.close()
 
 
